@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --gpus 1 --steps K --warmup W      # the reference path on the host CPU cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    # + what the last timed step computed, DIR/*.npy
 
 Workload (BASELINE.json): MF-ViT CA = two ViT-S/16 branches (CXR + enhanced CXR) + CLS cross-attention fusion + two summed
 aux heads, 224x224 synthetic CXR tensors, random-init weights.  N=1: configs[1] (32 pairs); N>1: configs[2] (64 pairs per
@@ -358,6 +359,27 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+DUMP_SAMPLE = 1 << 22  # parameters kept per encoder by --dump-outputs: 16 MB of its 87 MB
+
+
+def dump_step_outputs(out_dir, trainer, loss, fus, cxr, enh):
+    """--dump-outputs: what one training step hands its caller, as float32 .npy files - the loss, the three logit sets
+    (fused, CXR head, enhanced head) and the parameters after the optimizer step: every one of the fusion's, and a fixed
+    seeded sample of DUMP_SAMPLE of each encoder's (module.parameters() order, flattened), so that the files of two builds
+    run with the same arguments compare element for element."""
+    import numpy as np
+    fused, x_c, x_e = trainer.logits()
+    out = {"loss": loss, "logits_fused": fused, "logits_cxr": x_c, "logits_enh": x_e,
+           "params_fusion": torch.cat([p.detach().reshape(-1) for p in fus.parameters()])}
+    for name, m in (("cxr", cxr), ("enh", enh)):
+        flat = torch.cat([p.detach().reshape(-1) for p in m.parameters()])
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+        out["params_%s_sample" % name] = flat[torch.from_numpy(idx).to(flat.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def workload_config(args, per_gpu):
     return {
         "workload": "MF-ViT CA: 2x ViT-S/16 (CXR + enhanced) + CLS cross-attention fusion + 2 summed aux heads, "
@@ -386,7 +408,13 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip the stock-PyTorch GPU baseline leg (N = 1)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying the "
                                                             "CUDA graph of the step (single-GPU runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (loss, "
+                                                          "logits, parameters after the step) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "mfvit":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl mfvit)")
     if args.warmup < 3 and args.impl == "mfvit":
         args.warmup = 3
     if args.pairs_per_gpu <= 0:
@@ -471,6 +499,8 @@ def main():
     end.record()
     barrier()
     elapsed_ms = start.elapsed_time(end)
+    if args.dump_outputs and rank == 0:
+        dump_step_outputs(args.dump_outputs, trainer, loss, fus, cxr, enh)
     # kernels of libmfvit.so per step: eager launches are counted by the library, graph replays re-issue the launches
     # counted while the step was captured
     launches = (lib.mfv_launch_count() + trainer.graph_replays * trainer.graph_launches - launches0) / args.steps

@@ -7,9 +7,6 @@ modules INTEGRATION.md section 2 lists (vits.py, vits_returnftrs.py, model/modul
 moco/builder_vit_mocov3structure_mocov2loss[_noprediction_q].py) by the ones of dropin/.  Everything else of the
 reference - the main_*.py scripts, moco/loader.py, aihc_utils, training_tools, config - stays as it is, and the scripts
 run unmodified (tests/test_reference_loop.py executes MAIN_CA's own train() that way).
-
-`stage_reference()` is the recipe behind baseline/_ref/reference (git-ignored, travels to the GPU box): an unmodified
-copy of the reference tree, taken by __graft_entry__.build() whenever /root/reference is present.
 """
 import os
 import shutil
@@ -18,18 +15,6 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 DROPIN = os.path.join(PKG, "dropin")
-ROOT = os.path.dirname(PKG)
-STAGED = os.path.join(ROOT, "baseline", "_ref", "reference")
-
-
-def stage_reference(src="/root/reference", dst=STAGED):
-    """Unmodified copy of the reference tree (Python sources only: 25 files) for tests that drive its own code."""
-    if not os.path.isdir(src):
-        return None
-    if os.path.isdir(dst):
-        shutil.rmtree(dst)
-    shutil.copytree(src, dst, ignore=shutil.ignore_patterns(".git", "__pycache__", "*.pyc"))
-    return dst
 
 
 def make_overlay(reference_root, dest):

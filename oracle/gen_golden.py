@@ -1,6 +1,6 @@
-"""Generates tests/golden/*.pt by running the REAL reference modules (imported from /root/reference) on seeded inputs.
+"""Generates tests/golden/*.pt by running the REAL reference modules on seeded inputs.
 
-    python oracle/gen_golden.py          # authoring container only
+    MFVIT_REFERENCE=/path/to/Multi-Feature-ViT python oracle/gen_golden.py
 
 Fixtures are kept small (reduced width / tiny ViT) so they can be committed; the restatement in oracle/ is
 width-agnostic, so pinning it at width 96 pins the code that the CUDA parity tests use at width 384."""
@@ -124,7 +124,7 @@ def gen_augment():
     import torchvision.transforms as T
     from PIL import Image
     spec = importlib.util.spec_from_file_location(
-        "ref_image_transform", "/root/reference/moco_pretraining/moco/aihc_utils/image_transform.py")
+        "ref_image_transform", os.path.join(ref_loader.REF_ROOT, "aihc_utils", "image_transform.py"))
     it = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(it)
     rng = np.random.default_rng(99)

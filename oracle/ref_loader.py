@@ -1,19 +1,20 @@
-"""Imports the REAL reference modules from /root/reference (authoring container only - the path does not exist on the
-GPU box).  Used by oracle/gen_golden.py to produce tests/golden/*.pt and by CPU tests that re-validate the restatement
-when the reference tree is present.  TEST INFRASTRUCTURE ONLY."""
+"""Imports the REAL reference modules from a checkout of endiqq/Multi-Feature-ViT named by the MFVIT_REFERENCE
+environment variable (the repository does not contain it).  Used by oracle/gen_golden.py to produce tests/golden/*.pt.
+TEST INFRASTRUCTURE ONLY."""
 import importlib
 import os
 import sys
 import types
 
-REF_ROOT = "/root/reference/moco_pretraining/moco"
+REFERENCE = os.environ.get("MFVIT_REFERENCE", "")
+REF_ROOT = os.path.join(REFERENCE, "moco_pretraining", "moco") if REFERENCE else ""
 FUS_MODULE = ("model.crossvit_2vits_2additionaloutputs_changenormlayer_location_removeextralclayer_"
               "changemodelinputlocation_std002_sum")
 BLD_MODULE = "moco.builder_vit_mocov3structure_mocov2loss"
 
 
 def available():
-    return os.path.isdir(REF_ROOT)
+    return bool(REF_ROOT) and os.path.isdir(REF_ROOT)
 
 
 def _install_timm_shim():
@@ -55,7 +56,7 @@ class _RefPath:
 def load_reference():
     """Returns (module_py, fus_py, bld_py): the real MOD, FUS and BLD modules."""
     if not available():
-        raise RuntimeError("reference tree not present at %s" % REF_ROOT)
+        raise RuntimeError("reference tree not found: set MFVIT_REFERENCE to a checkout of endiqq/Multi-Feature-ViT")
     _install_timm_shim()
     with _RefPath():
         mod = importlib.import_module("model.module")

@@ -186,46 +186,46 @@ def test_cosine_momentum_schedule():
     assert 0.99 < moco_ref.cosine_momentum(50.0, 100, 0.99) < 1.0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="needs the reference tree (authoring container)")
-def test_whole_model_moco_restatement_equals_the_real_reference_class():
-    """oracle/moco_ref.MoCoViT (used by the GPU parity tests as the MoCo step oracle) against the REAL MoCo_ViT.forward
-    of BLD on the same tiny encoder, seed and inputs: logits, labels, queue and pointer are identical (the reference's
-    batch shuffle permutes which rows share nothing at one rank, so results agree exactly)."""
+def test_whole_model_moco_restatement_equals_the_real_reference_class(moco_golden):
+    """oracle/moco_ref.MoCoViT (used by the GPU parity tests as the MoCo step oracle) against the REAL MoCo_ViT of BLD:
+    tests/golden/moco_ref.pt records one train-mode forward of the real class on a tiny encoder (oracle/gen_golden.py
+    gen_moco: seed, construction, base-encoder perturbation, inputs).  Rebuilt from the same seed, the restatement must
+    draw the same weights and queue and reproduce every recorded output: predictor outputs, logits, labels, loss,
+    enqueued keys, pointer and the EMA (bit-exact).  The reference's key-batch shuffle (BLD:171) only permutes rows at
+    one rank, so results agree."""
     from functools import partial
-    from types import SimpleNamespace
-
-    import torch.distributed as dist
-    from oracle import ref_loader
-    _, _, bld_py = ref_loader.load_reference()
-    if not dist.is_initialized():
-        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-        os.environ.setdefault("MASTER_PORT", "29541")
-        dist.init_process_group("gloo", rank=0, world_size=1)
-    saved_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self, *a, **k: self  # BLD:121,194 hard-code .cuda()
-    try:
-        factory = partial(vit_ref.VisionTransformerMoCo, img_size=32, patch_size=16, embed_dim=64, depth=2, num_heads=2)
-        torch.manual_seed(77)
-        real = bld_py.MoCo_ViT(factory, SimpleNamespace(arch="vit_tiny"), 32, 48, 0.2)
-        mine = moco_ref.MoCoViT(factory, 32, 48, 0.2)
-        mine.load_state_dict(real.state_dict(), strict=True)
-        with torch.no_grad():
-            for a, b in zip(real.base_encoder.parameters(), mine.base_encoder.parameters()):
-                d = torch.randn_like(a) * 0.01
-                a.add_(d)
-                b.add_(d)
-        real.eval(), mine.eval()  # running statistics: the shuffle of BLD:171 cannot change anything
-        im_q, im_k = torch.randn(8, 3, 32, 32), torch.randn(8, 3, 32, 32)
-        for step in range(2):
-            lr, yr = real(im_q, im_k, 0.99)
-            lm, ym = mine(im_q, im_k, 0.99)
-            assert torch.allclose(lr, lm, atol=1e-6), float((lr - lm).abs().max())
-            assert torch.equal(yr, ym) and int(real.queue_ptr) == int(mine.queue_ptr) == 8 * (step + 1)
-            assert torch.allclose(real.queue, mine.queue, atol=1e-7)
-            for a, b in zip(real.momentum_encoder.parameters(), mine.momentum_encoder.parameters()):
-                assert torch.equal(a, b)  # EMA bit-exact
-    finally:
-        torch.Tensor.cuda = saved_cuda
+    g = moco_golden
+    factory = partial(vit_ref.VisionTransformerMoCo, img_size=32, patch_size=16, embed_dim=64, depth=2, num_heads=2)
+    torch.manual_seed(g["seed"])
+    mine = moco_ref.MoCoViT(factory, g["dim"], 48, g["T"])
+    assert mine.K == g["K"] and sum(p.numel() for p in mine.base_encoder.parameters()) == g["n_base"]
+    q0 = mine.queue.double()
+    assert (float(q0.sum()), float(q0.abs().sum())) == pytest.approx(g["queue_checksum"], rel=1e-12)
+    assert torch.equal(mine.queue[:, ::4096], g["queue_cols"])
+    with torch.no_grad():  # make base != momentum so the EMA is non-trivial
+        for p in mine.base_encoder.parameters():
+            p.add_(torch.randn_like(p) * 0.01)
+    im_q, im_k = torch.randn(8, 3, 32, 32), torch.randn(8, 3, 32, 32)
+    for a, b in zip(mine.momentum_encoder.parameters(), g["ema_before"]):
+        assert torch.equal(a, b)
+    for a, b in zip(mine.base_encoder.parameters(), g["ema_q"]):
+        assert torch.equal(a, b)
+    mine.train()
+    raw = []
+    h = mine.predictor.register_forward_hook(lambda mod, i, o: raw.append(o.detach().clone()))
+    logits, labels = mine(im_q, im_k, g["m"])
+    h.remove()
+    assert torch.allclose(raw[0], g["q_raw"], atol=1e-6) and torch.allclose(raw[1], g["k_raw"], atol=1e-6)
+    logits = logits.detach()
+    assert torch.allclose(logits[:, :65], g["logits_head"], atol=1e-6), float((logits[:, :65] - g["logits_head"]).abs().max())
+    assert torch.allclose(logits[:, 1::4096], g["logits_sampled"], atol=1e-6)
+    assert torch.allclose(torch.logsumexp(logits, dim=1), g["lse"], atol=1e-6)  # every column of the 65 537
+    assert abs(float(F.cross_entropy(logits, labels)) - float(g["loss"])) < 1e-6
+    assert torch.equal(labels, g["labels"]) and int(mine.queue_ptr) == int(g["queue_ptr_after"]) == 8
+    assert torch.allclose(mine.queue[:, :8], g["enqueued"], atol=1e-7)
+    assert torch.equal(mine.queue[:, 4096::4096], g["queue_cols"][:, 1:])  # columns past the pointer untouched
+    for a, b in zip(mine.momentum_encoder.parameters(), g["ema_after"]):
+        assert torch.equal(a, b)  # EMA bit-exact
 
 
 def test_pos_embed_against_an_independent_hand_written_sincos():
