@@ -35,9 +35,20 @@ int mfv_init(int device);
 const char* mfv_strerror(int code);
 /* "file:line: expression" of the last CUDA runtime failure returned to this thread ("" if none); debugging aid. */
 const char* mfv_last_error_where(void);
-/* Runtime switches (A/B measurements, tests): key in {"pdl", "side_stream", "legacy_attention", "rows96", "fuse_ln"};
- * the defaults come from the environment (MFVIT_PDL=0, MFVIT_SIDE_STREAM=0, MFVIT_ATTN=legacy, MFVIT_ROWS96=1,
- * MFVIT_FUSE_LN=0).                                                                                                 */
+/* Runtime switches (A/B measurements, tests).  Each key starts from its environment variable, read on first use; the
+ * value in brackets is the default when that variable is unset.  Returns MFV_ERR_ARG for an unknown key.
+ *   "pdl"              programmatic dependent launch                          [1]  MFVIT_PDL=0 switches it off
+ *   "side_stream"      weight gradients on a second stream                    [1]  MFVIT_SIDE_STREAM=0
+ *   "legacy_attention" mma.sync attention kernels instead of tcgen05          [0]  MFVIT_ATTN=legacy
+ *   "rows96"           192-row pair tiles for the forward N = 384 GEMMs       [0]  MFVIT_ROWS96=<digit>
+ *   "fuse_ln"          LayerNorm inside the proj / fc2 epilogues              [1]  MFVIT_FUSE_LN=0
+ *   "dx32"             fp32 residual-gradient stream in the backward          [0]  MFVIT_DX32=1
+ *   "patch_tma"        im2col-free patch-embedding GEMM (TMA from the images) [1]  MFVIT_PATCH_TMA=0
+ *   "reserve_sms"      SMs left free for concurrent collectives               [0]  MFVIT_RESERVE_SMS=<n>
+ *   "gemm_mc"          B-operand multicast between CTA pairs                  [0]  MFVIT_GEMM_MC=1
+ *   "streamk"          stream-K bit mask of GEMM families (allocates; not
+ *                      inside a stream capture)                               [0]  MFVIT_STREAMK=<mask>
+ *   "streamk_min_kb"   fewest k-blocks per stream-K range                     [12] MFVIT_STREAMK_MINKB=<n>   */
 int mfv_set_option(const char* key, int value);
 int mfv_num_sms(void);
 /* Number of kernels this library has launched so far in the process (bench.py reports the per-step delta). */
