@@ -373,6 +373,37 @@ int mfv_adam_step_dev(float* p, const float* g, float* exp_avg, float* exp_avg_s
                       int64_t n, const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
                       int decoupled_wd, const int64_t* step_dev, void* stream);
 
+/* ---- LARS (MoCo-v3 optimizer) -------------------------------------------------------------------------------------
+ * Replaces moco/optimizer.py:10-43 (LARS.step over every parameter with a gradient), built at MAIN_PRE:334-345 and
+ * stepped at MAIN_PRE:547.  Per tensor, with eta = trust_coefficient:
+ *   trust (ndim > 1): dp = g + wd*p ; q = (||p|| > 0 && ||dp|| > 0) ? eta*||p||/||dp|| : 1 ; dp *= q
+ *   else            : dp = g                          (no weight decay, no trust ratio)
+ *   mu = momentum*mu + dp ; p -= lr*mu                 (mu starts at zero; the 16-bit shadows are rewritten from p)
+ * Frozen tensors are simply not in the table.  The table lives in device memory and is built once by the caller: one
+ * record per tensor, every tensor split into chunks of MFV_LARS_CHUNK elements, chunk0 = the sum of
+ * ceil(n / MFV_LARS_CHUNK) over the records before it (ascending), n_chunks = the total.  p, g, mu 16-byte aligned,
+ * shadows 8-byte aligned (any n).  Two launches: the first writes per-chunk fp32 partial sums of p^2 and
+ * dp^2 of the trust tensors into `workspace` (mfv_lars_workspace_bytes); in the second every chunk sums its tensor's partials in a fixed tree,
+ * forms q (also stored in q_out f32 [n_tensors] when not NULL; 1 for the other tensors) and updates mu, p and the
+ * shadows.  No atomics: bit-identical results for the same table and state.  lr_dev f32 [1] (the schedule, read on the
+ * device, so a captured step follows it).                                                                            */
+#define MFV_LARS_CHUNK 32768
+typedef struct {
+  float* p;
+  const float* g;
+  float* mu;
+  void* shadow_bf16; /* NULL or bf16 [n] */
+  void* shadow_f16;  /* NULL or fp16 [n] */
+  int64_t n;
+  int64_t chunk0;
+  int32_t trust;     /* 1: ndim > 1 */
+  int32_t reserved;
+} mfv_lars_tensor;
+size_t mfv_lars_workspace_bytes(int64_t n_chunks);
+int mfv_lars_step_dev(const mfv_lars_tensor* table_dev, int64_t n_tensors, int64_t n_chunks, float* workspace,
+                      float* q_out, const float* lr_dev, float momentum, float weight_decay, float trust_coefficient,
+                      void* stream);
+
 /* ---- paired input pipeline, device side (SURVEY 8(f) row 3) -----------------------------------------------------------
  * Replaces the per-sample torchvision transform of the training loaders (image_transform.py:50-84 composed at
  * MAIN_CA:524-531, applied at loader.py:127-129): RandomHorizontalFlip -> RandomRotation (nearest, Pillow's 16.16

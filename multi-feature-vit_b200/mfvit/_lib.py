@@ -48,6 +48,14 @@ class EmaChunk(C.Structure):
     _fields_ = [("k", c_vp), ("q", c_vp), ("n", i64)]
 
 
+class LarsTensor(C.Structure):
+    _fields_ = [("p", c_vp), ("g", c_vp), ("mu", c_vp), ("shadow_bf16", c_vp), ("shadow_f16", c_vp), ("n", i64),
+                ("chunk0", i64), ("trust", i32), ("reserved", i32)]
+
+
+LARS_CHUNK = 32768  # MFV_LARS_CHUNK
+
+
 class VitPlan(C.Structure):
     _fields_ = (
         [(n, i64) for n in ["G", "B", "S", "C", "H", "depth", "hidden", "img", "np", "P"]]
@@ -123,6 +131,8 @@ SIGNATURES = {
     "mfv_adam_step": (C.c_int, [c_vp] * 6 + [i64, f32, f32, f32, f32, f32, C.c_int, i64, c_vp]),
     "mfv_sgd_step_dev": (C.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, i64, c_vp, f32, f32, C.c_int, c_vp]),
     "mfv_adam_step_dev": (C.c_int, [c_vp] * 6 + [i64, c_vp, f32, f32, f32, f32, C.c_int, c_vp, c_vp]),
+    "mfv_lars_workspace_bytes": (C.c_size_t, [i64]),
+    "mfv_lars_step_dev": (C.c_int, [c_vp, i64, i64, c_vp, c_vp, c_vp, f32, f32, f32, c_vp]),
 }
 
 _lib = None

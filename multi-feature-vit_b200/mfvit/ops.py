@@ -5,8 +5,8 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import (EPI_ATOMIC_F32, EPI_BF16, EPI_DGELU, EPI_F32, EPI_GELU, EPI_RESID_F32, EPI_RESID_LN, EmaChunk, FusionGrads,
-                   FusionParams, GemmArgs, MfvError, check)
+from ._lib import (EPI_ATOMIC_F32, EPI_BF16, EPI_DGELU, EPI_F32, EPI_GELU, EPI_RESID_F32, EPI_RESID_LN, LARS_CHUNK,
+                   EmaChunk, FusionGrads, FusionParams, GemmArgs, LarsTensor, MfvError, check)
 
 
 def _lib_for(t):
@@ -457,6 +457,63 @@ def adam_step_dev_(p, g, m1, m2, shadow, lr_dev, betas, eps, weight_decay, decou
     check(_lib_for(p).mfv_adam_step_dev(_p(p), _p(g), _p(m1), _p(m2), _p(shadow), _p(shadow16), p.numel(), _p(lr_dev),
                                         float(betas[0]), float(betas[1]), float(eps), float(weight_decay),
                                         int(bool(decoupled)), _p(step_dev), _stream()), "mfv_adam_step_dev")
+
+
+def make_lars_table(records, device):
+    """records: list of (p, g, mu, shadow_bf16 | None, shadow_f16 | None, trust) with p, g, mu contiguous fp32 CUDA
+    tensors of one size (16-byte aligned) and the shadows bf16 / fp16 of that size (8-byte aligned); trust = the
+    tensor is a matrix (ndim > 1).  Returns (table_dev uint8, n_tensors, n_chunks).  The table holds raw pointers: the
+    caller keeps every tensor alive (and in place) for as long as it steps with the table."""
+    arr = (LarsTensor * len(records))()
+    chunk = 0
+    for i, (p, g, mu, sb, sh, trust) in enumerate(records):
+        n = p.numel()
+        for t, what in ((p, "p"), (g, "g"), (mu, "mu")):
+            _lib_for(t)
+            if t.dtype != torch.float32 or t.numel() != n or not t.is_contiguous() or t.device != p.device:
+                raise MfvError("make_lars_table: record %d: %s must be a contiguous fp32 tensor of %d elements on %s"
+                               % (i, what, n, p.device))
+            if t.data_ptr() & 15:
+                raise MfvError("make_lars_table: record %d: %s is not 16-byte aligned" % (i, what))
+        for t, dt, what in ((sb, torch.bfloat16, "shadow_bf16"), (sh, torch.float16, "shadow_f16")):
+            if t is None:
+                continue
+            _lib_for(t)
+            if t.dtype != dt or t.numel() != n or not t.is_contiguous() or t.device != p.device:
+                raise MfvError("make_lars_table: record %d: %s must be a contiguous %s tensor of %d elements on %s"
+                               % (i, what, dt, n, p.device))
+            if t.data_ptr() & 7:
+                raise MfvError("make_lars_table: record %d: %s is not 8-byte aligned" % (i, what))
+        if n == 0:
+            raise MfvError("make_lars_table: record %d is empty" % i)
+        r = arr[i]
+        r.p, r.g, r.mu = p.data_ptr(), g.data_ptr(), mu.data_ptr()
+        r.shadow_bf16 = sb.data_ptr() if sb is not None else None
+        r.shadow_f16 = sh.data_ptr() if sh is not None else None
+        r.n, r.chunk0, r.trust = n, chunk, int(bool(trust))
+        chunk += (n + LARS_CHUNK - 1) // LARS_CHUNK
+    host = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8)
+    return host.to(device), len(records), chunk
+
+
+def lars_workspace(n_chunks, device):
+    n = _lib.load().mfv_lars_workspace_bytes(int(n_chunks))
+    return torch.empty(max(n // 4, 2), device=device, dtype=torch.float32)
+
+
+def lars_step_dev_(table_dev, n_tensors, n_chunks, workspace, lr_dev, momentum, weight_decay, trust_coefficient,
+                   q_out=None):
+    """LARS step (moco/optimizer.py:10-43) over every tensor of a make_lars_table() table, learning rate read from the
+    device tensor lr_dev f32 [1]; q_out (optional) f32 [n_tensors] receives the trust ratio of each tensor (1 for
+    vectors and for matrices with a zero norm)."""
+    lib = _lib_for(table_dev)
+    if workspace.numel() * 4 < lib.mfv_lars_workspace_bytes(int(n_chunks)) or workspace.dtype != torch.float32:
+        raise MfvError("lars_step_dev_: the workspace holds fewer than the %d chunks' partial sums" % n_chunks)
+    if q_out is not None and (q_out.dtype != torch.float32 or q_out.numel() < n_tensors or not q_out.is_contiguous()):
+        raise MfvError("lars_step_dev_: q_out must be a contiguous fp32 tensor of at least %d elements" % n_tensors)
+    check(lib.mfv_lars_step_dev(_p(table_dev), int(n_tensors), int(n_chunks), _p(workspace), _p(q_out), _p(lr_dev),
+                                float(momentum), float(weight_decay), float(trust_coefficient), _stream()),
+          "mfv_lars_step_dev")
 
 
 def adam_step_(p, g, m1, m2, shadow, lr, betas, eps, weight_decay, decoupled, step, shadow16=None):

@@ -14,7 +14,10 @@ What changes against the reference's loop body:
     run under bf16 autocast, so nothing can underflow the way fp16 gradients do (SURVEY 8(f) row 1);
   * `torch.optim.AdamW` over ~170 tensors becomes the fused flat-buffer AdamW (mfv_adam_step_dev): one launch for the
     encoder's flat master (which also rewrites the 16-bit GEMM shadows, so the next forward skips the cast pass) and one
-    for the packed projector + predictor parameters; the learning rate and step count live on the device;
+    for the packed projector + predictor parameters; the learning rate and step count live on the device.  The other
+    two optimizers MAIN_PRE:334-345 offers run the same way: optimizer='adam' (torch.optim.Adam, L2 weight decay) and
+    optimizer='lars' (moco/optimizer.py, the script's argparse default, MAIN_PRE:131): two launches of mfv_lars_step_dev
+    over a table of every trainable tensor - the per-tensor trust ratios are formed on the device;
   * the cosine learning rate with warm-up and the cosine momentum (MAIN_PRE:608-629) come from mfvit.schedules.
 DistributedDataParallel keeps doing the gradient all-reduce (bucketed NCCL, overlapped with the backward) and
 SyncBatchNorm the global statistics, exactly as MAIN_PRE:297,312 set them up.
@@ -30,7 +33,14 @@ from .trainer import FlatParams
 
 class MoCoPretrainer:
     def __init__(self, model, lr, weight_decay=0.1, betas=(0.9, 0.999), eps=1e-8, epochs=100, warmup_epochs=0,
-                 moco_m=0.99, moco_m_cos=True, cos=True, schedule=(), autocast_dtype=torch.bfloat16, fast_syncbn=True):
+                 moco_m=0.99, moco_m_cos=True, cos=True, schedule=(), autocast_dtype=torch.bfloat16, fast_syncbn=True,
+                 optimizer="adamw", momentum=0.9, trust_coefficient=0.001):
+        """optimizer: "adamw" (torch.optim.AdamW, MAIN_PRE:339; betas, eps), "adam" (torch.optim.Adam with L2 weight
+        decay; betas, eps) or "lars" (moco/optimizer.py LARS: momentum, trust_coefficient; matrices get weight decay and
+        the trust ratio, vectors momentum only).  weight_decay applies to all three."""
+        if optimizer not in ("adamw", "adam", "lars"):
+            raise MfvError("optimizer must be 'adamw', 'adam' or 'lars', not %r" % (optimizer,))
+        self.optimizer, self.momentum, self.trust_coefficient = optimizer, float(momentum), float(trust_coefficient)
         # nn.SyncBatchNorm (MAIN_PRE:297) -> the lean implementation sharing its tensors (mfvit/syncbn.py): same numbers,
         # one collective per call, a tenth of the host time; fast_syncbn=False keeps the stock modules
         self.swapped_syncbn = 0
@@ -62,8 +72,13 @@ class MoCoPretrainer:
         for p, gv in zip(rest, self._small.gviews):
             p.grad = gv  # autograd (and DDP's bucket copy-back) accumulate in place into the packed gradient buffer
         z = torch.zeros_like
-        self._m1_e, self._m2_e = z(eng.master), z(eng.master)
-        self._m1_s, self._m2_s = z(self._small.master), z(self._small.master)
+        if self.optimizer == "lars":
+            self._mu_e, self._mu_s = z(eng.master), z(self._small.master)
+            self._lars_tables = {}
+            self._lars_ws = self.lars_q = None
+        else:
+            self._m1_e, self._m2_e = z(eng.master), z(eng.master)
+            self._m1_s, self._m2_s = z(self._small.master), z(self._small.master)
         self._lr_dev = torch.full((1,), self.lr, device=device, dtype=torch.float32)
         self._step_dev = torch.zeros(1, device=device, dtype=torch.int64)
         self._loss_sum = torch.zeros(1, device=device, dtype=torch.float64)
@@ -114,23 +129,65 @@ class MoCoPretrainer:
             loss = F.cross_entropy(logits.float(), labels)              # MAIN_PRE:535
         loss.backward()                                                 # DDP all-reduces bucket by bucket
         grad = self._flat_encoder_grad()
-        self._step_dev.add_(1)
-        for lo, hi in self._runs:                                       # MAIN_PRE:547: AdamW, fused over the flat buffers
-            sl = slice(lo, hi)
-            ops.adam_step_dev_(eng.master[0, sl], grad[0, sl], self._m1_e[0, sl], self._m2_e[0, sl], eng.shadow[0, sl],
-                               self._lr_dev, self.betas, self.eps, self.wd, True, self._step_dev,
-                               shadow16=eng.shadow16[0, sl] if eng.fwd_f16 else None)
+        lars = self.optimizer == "lars"
+        decoupled = self.optimizer == "adamw"
+        if lars:                                                        # MAIN_PRE:547: LARS, encoder + projector + predictor
+            table, n_tensors, n_chunks = self._lars_table(grad)
+            ops.lars_step_dev_(table, n_tensors, n_chunks, self._lars_ws, self._lr_dev, self.momentum, self.wd,
+                               self.trust_coefficient, q_out=self.lars_q)
+        else:
+            self._step_dev.add_(1)
+            for lo, hi in self._runs:                                   # MAIN_PRE:547: AdamW, fused over the flat buffers
+                sl = slice(lo, hi)
+                ops.adam_step_dev_(eng.master[0, sl], grad[0, sl], self._m1_e[0, sl], self._m2_e[0, sl],
+                                   eng.shadow[0, sl], self._lr_dev, self.betas, self.eps, self.wd, decoupled,
+                                   self._step_dev, shadow16=eng.shadow16[0, sl] if eng.fwd_f16 else None)
         if not self._shadow_complete:
             eng.cast_shadow()
             self._shadow_complete = True
         eng.mark_shadow_fresh()
         sm = self._small
-        ops.adam_step_dev_(sm.master, sm.grad, self._m1_s, self._m2_s, None, self._lr_dev, self.betas, self.eps, self.wd,
-                           True, self._step_dev)
+        if not lars:
+            ops.adam_step_dev_(sm.master, sm.grad, self._m1_s, self._m2_s, None, self._lr_dev, self.betas, self.eps,
+                               self.wd, decoupled, self._step_dev)
         self._loss_sum += loss.detach().double() * im_q.shape[0]        # MAIN_PRE:537 without the .item()
         self._n_seen += im_q.shape[0]
         self.steps += 1
         return loss.detach()
+
+    def _lars_table(self, grad):
+        """The LARS tensor table for this gradient buffer (the engine alternates between two) and shadow format: one
+        record per trainable tensor of the encoder layout - frozen tensors (pos_embed, the conv under stop_grad_conv1)
+        and the alignment gaps between tensors are never touched - then one per projector / predictor tensor.  Built
+        once per buffer; self.lars_params lists the Parameters in table order, self.lars_q their trust ratios of the
+        last step (1 for vectors)."""
+        eng = self.engine
+        key = (grad.data_ptr(), eng.fwd_f16)
+        tab = self._lars_tables.get(key)
+        if tab is not None:
+            return tab
+        lay, sm = eng.layout, self._small
+        recs, params = [], []
+        for (name, shape, off), (_, p) in zip(lay.entries, eng._params[0]):
+            if p.requires_grad:
+                sl = slice(off, off + p.numel())
+                recs.append((eng.master[0, sl], grad[0, sl], self._mu_e[0, sl], eng.shadow[0, sl],
+                             eng.shadow16[0, sl] if eng.fwd_f16 else None, len(shape) > 1))
+                params.append(p)
+        base = sm.master.data_ptr()
+        for p, v, gv in zip(sm.params, sm.views, sm.gviews):
+            off = (v.data_ptr() - base) // 4
+            recs.append((v.view(-1), gv.view(-1), self._mu_s[off:off + v.numel()], None, None, v.dim() > 1))
+            params.append(p)
+        tab = ops.make_lars_table(recs, grad.device)
+        if self._lars_ws is None:
+            self._lars_ws = ops.lars_workspace(tab[2], grad.device)
+            self.lars_q = torch.ones(tab[1], device=grad.device, dtype=torch.float32)
+        if len(self._lars_tables) >= 4:  # gradient buffers replaced over time: keep the table cache small
+            self._lars_tables.clear()
+        self._lars_tables[key] = tab
+        self.lars_params = params
+        return tab
 
     def _flat_encoder_grad(self):
         """The engine's flat gradient buffer of this backward.  autograd normally adopts the views the encoder backward
