@@ -212,7 +212,9 @@ typedef struct {
 size_t mfv_fusion_saved_floats(int64_t B, int64_t S, int64_t C, int64_t heads);
 int mfv_fusion_fwd(const float* tok, const mfv_fusion_params* p, float* out_fused, float* out_x, float* saved,
                    int64_t B, int64_t S, int64_t C, int64_t heads, int64_t NC, void* stream);
-/* dtok f32 [2][B][S][C] is OVERWRITTEN (all rows); parameter gradients are accumulated (+=).                          */
+/* dtok f32 [2][B][S][C] is OVERWRITTEN (all rows); parameter gradients are accumulated (+=).  Where vhead_w[d] is NULL
+ * the vhead gradients of direction d are left untouched.  A backward issued while a deferred one is pending waits for
+ * its contraction before it writes anything.                                                                         */
 int mfv_fusion_bwd(const float* tok, const mfv_fusion_params* p, const float* saved, const float* d_fused,
                    const float* d_x, float* dtok, const mfv_fusion_grads* g, int64_t B, int64_t S, int64_t C,
                    int64_t heads, int64_t NC, void* stream);

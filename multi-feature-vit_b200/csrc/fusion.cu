@@ -111,11 +111,14 @@ __device__ __forceinline__ FusPtrs pick(const mfv_fusion_params& p, int d) {
 // Shared-memory vectors of the forward core (all length C unless noted)
 struct FusSmem {
   float *g1, *b1, *f0, *n0, *xh0, *q, *t /*heads*C*/, *u /*heads*C*/, *o, *c, *chat, *e;
-  float *merge;   // [FUS_WARPS][heads][C] per-warp partials
+  float *merge;   // [FUS_WARPS][merge_slots(heads)][C] per-warp partials
   float *stat;    // [FUS_WARPS][heads][2] (m, l) ; then [heads] lse at stat_lse
   float *lse;     // [heads]
   float *misc;    // [8]: rho0, rhoc, ...
 };
+// per-warp slots of the merge buffer: one per head in the forward; the backward kernel also parks its two LN1
+// weight-gradient partials (dg1, db1) there, so there are at least two even with one head
+__host__ __device__ constexpr int merge_slots(int heads) { return heads < 2 ? 2 : heads; }
 template <int CPL>
 __device__ __forceinline__ FusSmem carve(float* base, int heads) {
   constexpr int C = CPL * 32;
@@ -124,7 +127,7 @@ __device__ __forceinline__ FusSmem carve(float* base, int heads) {
   s.g1 = p; p += C; s.b1 = p; p += C; s.f0 = p; p += C; s.n0 = p; p += C; s.xh0 = p; p += C; s.q = p; p += C;
   s.t = p; p += heads * C; s.u = p; p += heads * C; s.o = p; p += C; s.c = p; p += C; s.chat = p; p += C;
   s.e = p; p += C;
-  s.merge = p; p += FUS_WARPS * heads * C;
+  s.merge = p; p += FUS_WARPS * merge_slots(heads) * C;
   s.stat = p; p += FUS_WARPS * MAX_HEADS * 2;
   s.lse = p; p += MAX_HEADS;
   s.misc = p; p += 8;
@@ -132,7 +135,7 @@ __device__ __forceinline__ FusSmem carve(float* base, int heads) {
 }
 template <int CPL>
 __host__ __device__ constexpr size_t fus_smem_floats(int heads) {
-  return (size_t)(CPL * 32) * (10 + 2 * heads) + (size_t)FUS_WARPS * heads * (CPL * 32) + FUS_WARPS * MAX_HEADS * 2 +
+  return (size_t)(CPL * 32) * (10 + 2 * heads) + (size_t)FUS_WARPS * merge_slots(heads) * (CPL * 32) + FUS_WARPS * MAX_HEADS * 2 +
          MAX_HEADS + 8;
 }
 
@@ -1338,8 +1341,9 @@ extern "C" int mfv_fusion_fwd(const float* tok, const mfv_fusion_params* p, floa
     return fus2_forward(tok, p, out_fused, out_x, saved, B, S, (int)heads, (int)NC, reinterpret_cast<cudaStream_t>(stream));
   const size_t smem = fus_smem_floats<12>((int)heads) * sizeof(float);
   static bool attr = false;
-  if (!attr) {
-    MFV_CUDA_CHECK(cudaFuncSetAttribute(fusion_fwd_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (!attr) {  // opt in once for the largest head count, so a later call with more heads still launches
+    MFV_CUDA_CHECK(cudaFuncSetAttribute(fusion_fwd_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)(fus_smem_floats<12>(MAX_HEADS) * sizeof(float))));
     attr = true;
   }
   const float scale = 1.0f / sqrtf((float)(C / heads));
@@ -1362,6 +1366,13 @@ static int fusion_bwd_impl(const float* tok, const mfv_fusion_params* p, const f
   if (B > 65535) return MFV_ERR_SHAPE;
   float* scratch = const_cast<float*>(saved);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  // A deferred contraction still in flight reads its records and accumulates into the gradients: everything this
+  // backward writes (records, and the gradients when it is not deferred) must wait for it.
+  if (g_fusion_wgrad_pending) MFV_CUDA_CHECK(cudaStreamWaitEvent(st, g_fusion_ss->fusion_done, 0));
+  // Without the backbone heads there is no x and so no gradient for their parameters, whatever d_x holds.
+  mfv_fusion_grads gg = *g;
+  for (int d = 0; d < 2; ++d)
+    if (!p->vhead_w[d]) gg.vhead_w[d] = gg.vhead_b[d] = nullptr;
   if (batched_fusion_enabled()) {
     const bool have_fwd = g_fus2_last.tok == tok && g_fus2_last.saved == saved && g_fus2_last.B == B &&
                           g_fus2_last.S == S && g_fus2_last.heads == heads;
@@ -1374,10 +1385,14 @@ static int fusion_bwd_impl(const float* tok, const mfv_fusion_params* p, const f
     int rc = fus2_backward_main(tok, p, scratch, d_fused, d_x, dtok, B, S, (int)heads, (int)NC, st);
     if (rc) return rc;
   } else {
-    const size_t smem = (fus_smem_floats<12>((int)heads) + (size_t)C * (6 + 2 * heads) + MAX_HEADS + 2 * MAX_NC) * sizeof(float);
+    auto smem_for = [&](int h) {
+      return (fus_smem_floats<12>(h) + (size_t)C * (6 + 2 * h) + MAX_HEADS + 2 * MAX_NC) * sizeof(float);
+    };
+    const size_t smem = smem_for((int)heads);
     static bool attr = false;
-    if (!attr) {
-      MFV_CUDA_CHECK(cudaFuncSetAttribute(fusion_bwd_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (!attr) {  // opt in once for the largest head count, so a later call with more heads still launches
+      MFV_CUDA_CHECK(cudaFuncSetAttribute(fusion_bwd_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem_for(MAX_HEADS)));
       attr = true;
     }
     const float scale = 1.0f / sqrtf((float)(C / heads));
@@ -1390,12 +1405,11 @@ static int fusion_bwd_impl(const float* tok, const mfv_fusion_params* p, const f
   SideStream* ss = defer ? side_stream() : nullptr;
   cudaStream_t sw = st;
   if (ss) {
-    if (g_fusion_wgrad_pending) MFV_CUDA_CHECK(cudaStreamWaitEvent(st, g_fusion_ss->fusion_done, 0));  // never two in flight
     MFV_CUDA_CHECK(cudaEventRecord(ss->fusion_fork, st));
     MFV_CUDA_CHECK(cudaStreamWaitEvent(ss->stream, ss->fusion_fork, 0));
     sw = ss->stream;
   }
-  fusion_wgrad_kernel<12><<<dim3((unsigned)(C / 4), 5, 2), FUS_THREADS, 0, sw>>>(scratch, d_fused, d_x, *g, (int)B,
+  fusion_wgrad_kernel<12><<<dim3((unsigned)(C / 4), 5, 2), FUS_THREADS, 0, sw>>>(scratch, d_fused, d_x, gg, (int)B,
                                                                                  (int)heads, (int)NC);
   MFV_LAUNCH_CHECK();
   if (ss) {
