@@ -155,6 +155,24 @@ int mfv_attn_bwd_ws(const void* qkv, int qkv_is_f16, const void* o, const void* 
                     void* dqkv, float* workspace, int64_t NB, int64_t S, int64_t H, int64_t D, float scale,
                     void* stream);
 
+/* ---- explain pass: attention maps and CLS attention rollout --------------------------------------------------------
+ * Replaces a forward hook on timm Attention's `attn.softmax(dim=-1)` (same math MOD:52-64): the fused attention never
+ * writes its probabilities, so they are recomputed from one block's stored qkv (bf16, or fp16 when qkv_is_f16)
+ * [NB][S][3][H][D], NB = G*B (the qkv GEMM's natural layout, one slot of mfv_vit_plan.qkv after a saving forward):
+ *   P[nb][h][i][j] = softmax_j(scale * q_i . k_j), the dot an fp32 FMA chain over exact 16-bit products, the row maximum
+ *   and sum computed by the kernel itself (two passes; the forward's lse is not read).
+ * Outputs, each optional (NULL = skip): probs f32 [NB][H][S][S]; head_mean f32 [NB][S][S] = (sum over h = 0..H-1 in
+ * that order) / H, deterministic (no atomics).  D in {32, 64}, 1 <= S <= 577, NB <= 65535, qkv 4-byte aligned;
+ * anything else returns MFV_ERR_SHAPE (MFV_ERR_ALIGN for a misaligned qkv).                                          */
+int mfv_attn_probs(const void* qkv, int qkv_is_f16, float* probs, float* head_mean, int64_t NB, int64_t S, int64_t H,
+                   int64_t D, float scale, void* stream);
+/* CLS attention rollout (Abnar & Zuidema 2020) over head means head_mean f32 [L][NB][S][S] (block l of the encoder at
+ * index l): A'_l = (mean_l + I) / 2, out f32 [NB][S] = e_0^T A'_{L-1} ... A'_0, evaluated as the row-vector chain
+ * v <- v A'_l from l = L-1 down to 0 in a fixed order (one CTA per image, deterministic).  out[:, 0] is the CLS entry,
+ * out[:, 1:] the patches in row-major grid order (the patch embedding's flatten(2)); the entries sum to 1 in exact
+ * arithmetic and are not renormalised.  1 <= S <= 1024, else MFV_ERR_SHAPE.                                          */
+int mfv_attn_rollout(const float* head_mean, float* out, int64_t L, int64_t NB, int64_t S, void* stream);
+
 /* ---- patch embedding -----------------------------------------------------------------------------------------------
  * Replaces timm PatchEmbed Conv2d(3,C,k=16,s=16)+flatten+transpose, cls-token concat and pos-embed add
  * (commented restatement FUS:197-221, crossvit.py:130-146; SURVEY K1).
@@ -226,6 +244,13 @@ int mfv_fusion_bwd_deferred(const float* tok, const mfv_fusion_params* p, const 
                             const float* d_x, float* dtok, const mfv_fusion_grads* g, int64_t B, int64_t S, int64_t C,
                             int64_t heads, int64_t NC, void* stream);
 int mfv_fusion_bwd_join(void* stream);
+/* Explain pass: the fusion's cross-attention probabilities, i.e. what a hook on CrossAttention's `attn` (MOD:123-137)
+ * would read.  probs f32 [B][2][heads][S]: direction d as in mfv_fusion_params; key 0 is the query's own CLS row and keys
+ * 1..S-1 the other branch's patches (torch.cat((cal_q, x_other)), FUS:58,61).  Computed from tok in fp32 as the forward
+ * does (LN1 eps 1e-5, q = Wq xh_0, t_h = Wk_h^T q_h, s_j = scale t_h . xh_j), then a two-pass softmax per head.  Reads
+ * only ln1_w, ln1_b, wq and wk of `p`.  2 <= S <= 2048, heads 1..4, C == 384, B <= 65535, else MFV_ERR_SHAPE.       */
+int mfv_fusion_attn(const float* tok, const mfv_fusion_params* p, float* probs, int64_t B, int64_t S, int64_t C,
+                    int64_t heads, void* stream);
 
 /* ---- small-N linear (classification heads, N <= 32) ------------------------------------------------------------------
  * Replaces `head = nn.Linear(384, 3)` (MAIN_CA:309-310, MAIN_LPFT:288) applied to the CLS row.

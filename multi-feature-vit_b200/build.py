@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "mfvit")
 LIB = os.path.join(OUT_DIR, "libmfvit.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["runtime.cu", "gemm.cu", "ln.cu", "attn.cu", "attn_tc.cu", "elementwise.cu", "lars.cu", "augment.cu", "fusion.cu", "infonce.cu", "patch_embed.cu", "vit.cu"]
+SOURCES = ["runtime.cu", "gemm.cu", "ln.cu", "attn.cu", "attn_tc.cu", "attn_maps.cu", "elementwise.cu", "lars.cu", "augment.cu", "fusion.cu", "infonce.cu", "patch_embed.cu", "vit.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "-diag-suppress", "550"]
 

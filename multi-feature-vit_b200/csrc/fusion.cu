@@ -1189,6 +1189,94 @@ fus2_bwd_row0_kernel(const mfv_fusion_params prm, const float* __restrict__ fwd,
   }
 }
 
+// ------------------------------------------------------------------------------------------------ attention maps
+// probs[b][d][h][j] = softmax_j(scale t_h . xh_j) of instance (b, d): the same LN1 / q / t / score steps as the forward
+// core, the scores kept in shared memory, then a two-pass softmax per head (one warp per head).  Explain pass only.
+__host__ __device__ constexpr size_t fus_attn_smem_floats(int C, int heads, int S) {
+  return (size_t)C * (5 + heads) + (size_t)heads * S;
+}
+template <int CPL>
+__global__ void __launch_bounds__(FUS_THREADS, 1)
+fusion_attn_kernel(const float* __restrict__ tok, const mfv_fusion_params prm, float* __restrict__ probs, int B, int S,
+                   int heads, float scale) {
+  constexpr int C = CPL * 32;
+  extern __shared__ __align__(16) float fsm[];
+  float* g1 = fsm;
+  float* b1 = g1 + C;
+  float* f0 = b1 + C;
+  float* xh0 = f0 + C;
+  float* q = xh0 + C;
+  float* t = q + C;           // [heads][C]
+  float* s = t + heads * C;   // [heads][S]
+  const int d = blockIdx.x, b = blockIdx.y;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int hd = C / heads;
+  const FusPtrs P = pick(prm, d);
+  const float* cls_row = tok + ((size_t)d * B + b) * S * C;
+  const float* other = tok + ((size_t)(1 - d) * B + b) * S * C;
+  for (int c = tid; c < C; c += FUS_THREADS) {
+    g1[c] = P.ln1_w[c];
+    b1[c] = P.ln1_b[c];
+    f0[c] = cls_row[c];
+  }
+  __syncthreads();
+  if (warp == 0) {
+    float v[CPL], n[CPL];
+    load_row<CPL>(v, f0, lane);
+    float rstd;
+    ln_stats<CPL>(v, n, 1e-5f, rstd);
+#pragma unroll
+    for (int i = 0; i < CPL; ++i) {
+      const int c = col_of<CPL>(i, lane);
+      xh0[c] = n[i] * g1[c] + b1[c];
+    }
+  }
+  __syncthreads();
+  matvec_rows<CPL>(P.wq, xh0, nullptr, q, warp, lane);
+  __syncthreads();
+  for (int c = tid; c < C; c += FUS_THREADS) {
+    for (int h = 0; h < heads; ++h) {
+      float acc = 0.f;
+      const float* wk = P.wk + (size_t)(h * hd) * C + c;
+#pragma unroll 16
+      for (int i = 0; i < hd; ++i) acc += __ldg(wk + (size_t)i * C) * q[h * hd + i];
+      t[h * C + c] = acc;
+    }
+  }
+  __syncthreads();
+  for (int j = warp; j < S; j += FUS_WARPS) {  // key 0: the query's own CLS row; keys 1..S-1: the other branch's patches
+    float v[CPL], xh[CPL];
+    load_row<CPL>(v, j == 0 ? f0 : other + (size_t)j * C, lane);
+    float rstd;
+    ln_stats<CPL>(v, xh, 1e-5f, rstd);
+#pragma unroll
+    for (int i = 0; i < CPL; ++i) {
+      const int c = col_of<CPL>(i, lane);
+      xh[i] = xh[i] * g1[c] + b1[c];
+    }
+    for (int h = 0; h < heads; ++h) {
+      const float sc = scale * dot_row<CPL>(xh, t + h * C, lane);
+      if (lane == 0) s[h * S + j] = sc;
+    }
+  }
+  __syncthreads();
+  if (warp < heads) {
+    float* sh = s + warp * S;
+    float m = -INFINITY;
+    for (int j = lane; j < S; j += 32) m = fmaxf(m, sh[j]);
+    m = warp_max(m);
+    float l = 0.f;
+    for (int j = lane; j < S; j += 32) {
+      const float e = __expf(sh[j] - m);
+      sh[j] = e;
+      l += e;
+    }
+    l = warp_sum(l);
+    float* out = probs + (((size_t)b * 2 + d) * heads + warp) * S;
+    for (int j = lane; j < S; j += 32) out[j] = __fdiv_rn(sh[j], l);
+  }
+}
+
 }  // namespace mfv
 
 extern "C" size_t mfv_fusion_saved_floats(int64_t B, int64_t S, int64_t C, int64_t heads) {
@@ -1438,5 +1526,19 @@ extern "C" int mfv_fusion_bwd_join(void* stream) {
   if (!g_fusion_wgrad_pending) return MFV_OK;
   MFV_CUDA_CHECK(cudaStreamWaitEvent(reinterpret_cast<cudaStream_t>(stream), g_fusion_ss->fusion_done, 0));
   g_fusion_wgrad_pending = false;
+  return MFV_OK;
+}
+
+extern "C" int mfv_fusion_attn(const float* tok, const mfv_fusion_params* p, float* probs, int64_t B, int64_t S,
+                               int64_t C, int64_t heads, void* stream) {
+  using namespace mfv;
+  if (!p || !tok || !probs || B <= 0 || B > 65535 || S < 2 || S > 2048 || heads <= 0 || heads > MAX_HEADS)
+    return MFV_ERR_SHAPE;
+  if (C != 384 || C % heads) return MFV_ERR_SHAPE;
+  const size_t smem = fus_attn_smem_floats((int)C, (int)heads, (int)S) * sizeof(float);  // < 48 KB for S <= 2048
+  const float scale = 1.0f / sqrtf((float)(C / heads));
+  fusion_attn_kernel<12><<<dim3(2, (unsigned)B), FUS_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
+      tok, *p, probs, (int)B, (int)S, (int)heads, scale);
+  MFV_LAUNCH_CHECK();
   return MFV_OK;
 }

@@ -9,16 +9,21 @@ The reference evaluates each backbone twice (FUS:128,131 / 133,135); with all dr
 same function, so each backbone runs once here (SURVEY fact 5)."""
 import os
 import sys
+from collections import namedtuple
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import _path  # noqa: E402,F401
 import torch  # noqa: E402
 import torch.nn as nn  # noqa: E402
-from mfvit import MfvError  # noqa: E402
+from mfvit import MfvError, explain  # noqa: E402
 from mfvit.engine import encode, engine_for  # noqa: E402
 from mfvit.functions import FusionFn  # noqa: E402
 from model.module import Attention, CrossAttention, FeedForward, PreNorm  # noqa: E402,F401
 from torch.nn.init import trunc_normal_  # noqa: E402  (timm.models.layers.trunc_normal_ in the reference, FUS:9)
+
+
+# Fus_CrossViT.explain: the three outputs of forward plus where both backbones and the fusion looked
+Explanation = namedtuple("Explanation", "fused x_cxr x_enh rollout cross maps")
 
 
 class MultiScaleTransformerEncoder(nn.Module):
@@ -103,10 +108,27 @@ class Fus_CrossViT(nn.Module):
                 outs.append(None)
         return fused, outs[0], outs[1]
 
-    def forward(self, vit_cxr, vit_enh, img_cxr, img_enh):
+    def _check_backbones(self, vit_cxr, vit_enh, what):
         if getattr(self.vit_features_cxr, "__self__", None) is not vit_cxr or \
                 getattr(self.vit_features_enh, "__self__", None) is not vit_enh:
-            raise MfvError("Fus_CrossViT.forward expects the same backbone modules it was constructed with "
-                           "(MAIN_CA:393,862)")
+            raise MfvError("Fus_CrossViT.%s expects the same backbone modules it was constructed with "
+                           "(MAIN_CA:393,862)" % what)
+
+    def forward(self, vit_cxr, vit_enh, img_cxr, img_enh):
+        self._check_backbones(vit_cxr, vit_enh, "forward")
         tok = encode(engine_for(vit_cxr, vit_enh), [img_cxr, img_enh])
         return self.fuse_tokens(tok, vit_cxr, vit_enh)
+
+    def explain(self, vit_cxr, vit_enh, img_cxr, img_enh, blocks=()):
+        """forward's outputs and where the model looked, from one saving pass of the grouped encoder that forward uses
+        (a branch's own single-branch engine would re-point its Parameters away from the buffer a trainer steps).
+        Returns Explanation(fused, x_cxr, x_enh, rollout f32 [2, B, S] (cxr, enh), cross f32 [B, 2, heads, S],
+        maps f32 [2, B, len(blocks), H, S, S] or None when `blocks` is empty).  cross[:, 0] is the CXR CLS querying
+        the ENH patches, cross[:, 1] the reverse; key 0 is the query's own CLS row.  Everything is detached."""
+        self._check_backbones(vit_cxr, vit_enh, "explain")
+        with torch.no_grad():
+            tok, maps, roll = explain.encoder_attention(engine_for(vit_cxr, vit_enh), [img_cxr, img_enh], blocks,
+                                                        rollout=True)
+            fused, x_cxr, x_enh = self.fuse_tokens(tok, vit_cxr, vit_enh)
+            cross = explain.fusion_attention(tok, self._fusion_params(vit_cxr, vit_enh)[0], self.heads)
+        return Explanation(fused, x_cxr, x_enh, roll, cross, maps)

@@ -13,7 +13,7 @@ from operator import mul
 import _path  # noqa: F401
 import torch
 import torch.nn as nn
-from mfvit import MfvError
+from mfvit import MfvError, explain
 from mfvit.engine import encode, engine_for
 from mfvit.functions import HeadFn
 
@@ -138,6 +138,24 @@ class VisionTransformerMoCo(nn.Module):
 
     def forward(self, x):
         return self.apply_head(self.features3D(x))
+
+    # ------------------------------------------------------------------------------------------------ explain pass
+    def attention_maps(self, x, blocks=None):
+        """Per-head attention probabilities f32 [B, len(blocks), H, S, S] of the given blocks (None: all of them), i.e.
+        what a hook on each Attention's softmax would record; row i is query token i (0 = CLS), patches in row-major
+        grid order.  Detached; works with or without grad mode."""
+        blocks = range(self.depth) if blocks is None else list(blocks)
+        _, maps, _ = explain.encoder_attention(engine_for(self), [x], blocks, rollout=False)
+        if maps is None:
+            S = self.patch_embed.num_patches + 1
+            return torch.empty(x.shape[0], 0, self.num_heads, S, S, device=x.device)
+        return maps[0]
+
+    def attention_rollout(self, x):
+        """CLS attention rollout f32 [B, S] over all blocks (head-averaged maps, identity added, Abnar & Zuidema
+        2020): entry 0 is the CLS token, entries 1.. the patches in row-major grid order.  Detached."""
+        _, _, roll = explain.encoder_attention(engine_for(self), [x], (), rollout=True)
+        return roll[0]
 
 
 def vit_small(**kwargs):

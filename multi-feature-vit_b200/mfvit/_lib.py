@@ -95,6 +95,8 @@ SIGNATURES = {
     "mfv_attn_bwd": (C.c_int, [c_vp, C.c_int] + [c_vp] * 5 + [i64, i64, i64, i64, f32, c_vp]),
     "mfv_attn_bwd_workspace_bytes": (C.c_size_t, [i64, i64, i64, i64]),
     "mfv_attn_bwd_ws": (C.c_int, [c_vp, C.c_int] + [c_vp] * 6 + [i64, i64, i64, i64, f32, c_vp]),
+    "mfv_attn_probs": (C.c_int, [c_vp, C.c_int, c_vp, c_vp, i64, i64, i64, i64, f32, c_vp]),
+    "mfv_attn_rollout": (C.c_int, [c_vp, c_vp, i64, i64, i64, c_vp]),
     "mfv_patchify": (C.c_int, [c_vp, c_vp, C.c_int, c_vp, i64, i64, c_vp]),
     "mfv_debug_patch_tma_probe": (C.c_int, [c_vp, c_vp, i64, i64, i64, i64, i64, c_vp]),
     "mfv_patch_embed_tma": (C.c_int, [c_vp, c_vp, c_vp, C.c_int, c_vp, c_vp, c_vp, c_vp, i64, i64, i64, i64, i64, c_vp]),
@@ -108,6 +110,7 @@ SIGNATURES = {
     "mfv_fusion_bwd_deferred": (C.c_int, [c_vp, C.POINTER(FusionParams), c_vp, c_vp, c_vp, c_vp, C.POINTER(FusionGrads),
                                  i64, i64, i64, i64, i64, c_vp]),
     "mfv_fusion_bwd_join": (C.c_int, [c_vp]),
+    "mfv_fusion_attn": (C.c_int, [c_vp, C.POINTER(FusionParams), c_vp, i64, i64, i64, i64, c_vp]),
     "mfv_linear_small_fwd": (C.c_int, [c_vp, i64, c_vp, c_vp, c_vp, i64, i64, i64, c_vp]),
     "mfv_linear_small_bwd": (C.c_int, [c_vp, i64, c_vp, c_vp, c_vp, i64, c_vp, c_vp, i64, i64, i64, c_vp]),
     "mfv_ce_small": (C.c_int, [c_vp] * 6 + [i64, i64, c_vp]),

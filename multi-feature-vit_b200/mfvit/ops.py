@@ -186,6 +186,68 @@ def attn_bwd(qkv, o, d_o, lse):
     return dqkv
 
 
+def _want(t, shape, dtype, device, what):
+    """Rejects an argument the kernel would misread: wrong device, dtype, shape or a non-contiguous layout."""
+    _lib_for(t)
+    if t.device != device or t.dtype != dtype or tuple(t.shape) != tuple(shape) or not t.is_contiguous():
+        raise MfvError("%s must be a contiguous %s tensor of shape %s on %s, got %s %s%s on %s"
+                       % (what, dtype, tuple(shape), device, t.dtype, tuple(t.shape),
+                          "" if t.is_contiguous() else " (non-contiguous)", t.device))
+
+
+def attn_probs(qkv, probs=None, head_mean=None):
+    """Attention probabilities of one encoder block, recomputed from its stored qkv (bf16 | fp16 [NB,S,3,H,D]):
+    probs f32 [NB,H,S,S] = softmax(q k^T / sqrt(D)) and / or head_mean f32 [NB,S,S] (their mean over heads), written
+    into the given tensors (at least one).  Returns (probs, head_mean)."""
+    _lib_for(qkv)
+    if qkv.dim() != 5 or qkv.shape[2] != 3 or qkv.dtype not in (torch.bfloat16, torch.float16) \
+            or not qkv.is_contiguous():
+        raise MfvError("attn_probs wants a contiguous bf16 / fp16 qkv tensor [NB,S,3,H,D], got %s %s"
+                       % (qkv.dtype, tuple(qkv.shape)))
+    NB, S, _, H, D = qkv.shape
+    if probs is None and head_mean is None:
+        raise MfvError("attn_probs: pass probs and / or head_mean")
+    if probs is not None:
+        _want(probs, (NB, H, S, S), torch.float32, qkv.device, "attn_probs: probs")
+    if head_mean is not None:
+        _want(head_mean, (NB, S, S), torch.float32, qkv.device, "attn_probs: head_mean")
+    check(_lib_for(qkv).mfv_attn_probs(_p(qkv), int(qkv.dtype == torch.float16), _p(probs), _p(head_mean), NB, S, H, D,
+                                       float(D) ** -0.5, _stream()), "mfv_attn_probs")
+    return probs, head_mean
+
+
+def attn_rollout(head_mean, out=None):
+    """CLS attention rollout: head_mean f32 [L,NB,S,S] (block l at index l) -> out f32 [NB,S] = e_0^T prod_l (A_l+I)/2,
+    from block L-1 down to 0."""
+    _lib_for(head_mean)
+    if head_mean.dim() != 4 or head_mean.shape[-1] != head_mean.shape[-2]:
+        raise MfvError("attn_rollout wants head means [L,NB,S,S], got %s" % (tuple(head_mean.shape),))
+    L, NB, S, _ = head_mean.shape
+    _want(head_mean, (L, NB, S, S), torch.float32, head_mean.device, "attn_rollout: head_mean")
+    if out is None:
+        out = torch.empty(NB, S, device=head_mean.device, dtype=torch.float32)
+    _want(out, (NB, S), torch.float32, head_mean.device, "attn_rollout: out")
+    check(_lib_for(head_mean).mfv_attn_rollout(_p(head_mean), _p(out), L, NB, S, _stream()), "mfv_attn_rollout")
+    return out
+
+
+def fusion_attn(tok, params, heads, out=None):
+    """Cross-attention probabilities of the fusion: tok f32 [2,B,S,C] (cxr, enh), params a fusion_param_struct() (only
+    LN1, wq and wk are read) -> f32 [B,2,heads,S]; key 0 is the query's own CLS row, keys 1.. the other branch's
+    patches."""
+    _lib_for(tok)
+    if tok.dim() != 4 or tok.shape[0] != 2:
+        raise MfvError("fusion_attn wants tokens [2,B,S,C], got %s" % (tuple(tok.shape),))
+    _, B, S, Cd = tok.shape
+    _want(tok, (2, B, S, Cd), torch.float32, tok.device, "fusion_attn: tok")
+    if out is None:
+        out = torch.empty(B, 2, heads, S, device=tok.device, dtype=torch.float32)
+    _want(out, (B, 2, heads, S), torch.float32, tok.device, "fusion_attn: out")
+    check(_lib_for(tok).mfv_fusion_attn(_p(tok), C.byref(params), _p(out), B, S, Cd, int(heads), _stream()),
+          "mfv_fusion_attn")
+    return out
+
+
 def colsum_bf16(x, out):
     G, rows, Cd = x.shape
     check(_lib_for(x).mfv_colsum_bf16(_p(x), _p(out), G, rows, Cd, out.stride(0) if out.dim() > 1 else 0, _stream()),
